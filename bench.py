@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path, one rank per GPU (torchrun for N>1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (NumPy restatement), rank 0 only
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed to DIR/<name>.npy
 
 Prints ONE JSON line (rank 0).  Metric: train frames/sec = global_batch * T / step_time (BASELINE.json).
  value        : inputs resident in HBM, whole step replayed as a CUDA graph, CUDA-event time, max over ranks
@@ -24,6 +25,30 @@ sys.path.insert(0, ROOT)
 
 METRIC = "train frames/sec (CDNA, 64x64, b32)"
 T_SEQ, H, W, MASKS, K_SCHED, ITER0 = 10, 64, 64, 10, 900.0, 6000
+DUMP_MAX_ELEMS = 1 << 22              # per dumped array: the three large ones stay under 64 MB together
+
+
+def dump_outputs(out_dir, model):
+    """Write what the last training step handed its caller to out_dir/<name>.npy (float32, float64 for the scalars): loss, psnr_all, the
+    predicted frames and states, and the updated parameters and the gradients in Chainer layout, every tensor flattened and concatenated
+    in sorted name order.  An array of more than DUMP_MAX_ELEMS elements is reduced to its elements at a fixed, seeded choice of flat
+    indices, so that two builds run with the same arguments can be compared element for element.  The comparison needs a tolerance: the
+    step adds fp32 partial sums with atomics, and Adam amplifies those last-bit differences over the steps."""
+    import numpy as np
+    import torch
+
+    def flat(d):
+        return np.concatenate([d[k].reshape(-1) for k in sorted(d)])
+    arrays = {"loss": np.float64(float(model.loss)), "psnr_all": np.float64(float(model.psnr_all)),
+              "gen_images": torch.stack(list(model.gen_images)).float().cpu().numpy(),
+              "gen_states": torch.stack(list(model.gen_states)).float().cpu().numpy(),
+              "params": flat(model.params()), "grads": flat(model.grads)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if a.size > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.RandomState(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -121,7 +146,7 @@ def run_reference(args, rank):
     adam = OM.Adam()
     batch = OM.concat_examples(OM.synthetic_sequences(1, T_SEQ, cfg))
     np.random.seed(99)
-    steps, warm = max(1, min(args.steps, 5)), max(1, min(args.warmup, 1))
+    steps, warm = args.steps, max(1, min(args.warmup, 1))
     for i in range(warm):
         OM.train_step(params, adam, batch, ITER0 + i, cfg)
     t0 = time.perf_counter()
@@ -174,7 +199,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--global-batch", type=int, default=0, help="strong scaling: fixed GLOBAL batch split over the ranks (BASELINE config 3: 256)")
     ap.add_argument("--no-extras", action="store_true", help="skip the DNA-op (config 4) and STP 128x128 (config 5) measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     if args.impl == "reference":
         return run_reference(args, rank)
@@ -234,6 +264,8 @@ def main():
     ms_per_step = ms / args.steps
     value = B * world * T / (ms_per_step * 1e-3)
     loss_now = float(model.loss)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model)
 
     # ---------------- end to end: H2D of the batch from pinned memory + step + D2H loss read, every step
     barrier(); torch.cuda.synchronize()
