@@ -275,7 +275,8 @@ int pivp_tc_conv_taps_multi_ln(const void* in_bf16, int in_cs, int B, int H, int
 int pivp_cast_bf16(const float* src, int s_cs, int s_co, void* dst_bf16, int d_cs, int d_co, long M, int C, int H, int W, int s2d, int cblk,
                    void* stream);
 size_t pivp_tc_wgrad_taps_workspace_bytes(int SB, int H, int W, int Cx, int N4, int ntaps);
-/* general weight-gradient GEMM: dW[n][t][c] += sum_p A[p][n] * X[p + (dy_t,dx_t)][coff_t + c]  (n < N4, t < ntaps, c < Cx) */
+/* general weight-gradient GEMM: dW[n][t][c] += sum_p A[p][n] * X[p + (dy_t,dx_t)][coff_t + c]  (n < N4, t < ntaps, c < Cx).
+ * dW and workspace must be 16-byte aligned (PIVP_EINVAL otherwise). */
 int pivp_tc_wgrad_taps(const void* a_bf16, int a_cs, const void* x_bf16, int x_cs, int SB, int H, int W, int Cx, int N4, int ntaps,
                        const int* dy, const int* dx, const int* coff, float* dW, void* workspace, size_t ws_bytes, void* stream);
 /* out[c] += sum_p src[p][c] over a bf16 (P, ld) matrix -- the ConvLSTM bias gradient from the stacked dG of all time steps.
@@ -284,7 +285,7 @@ int pivp_tc_colsum_bf16(const void* src_bf16, int ld, long P, int C, float* out,
 size_t pivp_tc_wgrad_workspace_bytes(int SB, int H, int W, int Cx, int N4);
 /* dW[n][tap][c] += sum over all SB images (time steps x batch) and pixels p of dG[p][n] * XH[p + tap - 2][c]   (D.5).
  * dg: (SB*H*W, N4) bf16; xh: NHWC bf16 with row stride xh_cs >= ceil(Cx/64)*64 (pad channels are ignored). Both operands are
- * read MN-major by tcgen05.mma straight from these NHWC tensors. */
+ * read MN-major by tcgen05.mma straight from these NHWC tensors.  dW and workspace must be 16-byte aligned (PIVP_EINVAL otherwise). */
 int pivp_tc_wgrad5x5(const void* dg_bf16, const void* xh_bf16, int xh_cs, int SB, int H, int W, int Cx, int N4, float* dW,
                      void* workspace, size_t ws_bytes, void* stream);
 

@@ -358,6 +358,9 @@ size_t pivp_tc_wgrad_taps_workspace_bytes(int SB, int H, int W, int Cx, int N4, 
 static int launch_wgrad(const void* dg_bf16, int dg_cs, const void* xh_bf16, int xh_cs, int SB, int H, int W, int Cx, int N4, int ntaps,
                         const int* dy, const int* dx, const int* coff, float* dW, void* workspace, size_t ws_bytes, void* stream, const char* who) {
     PIVP_REQUIRE(dg_bf16 && xh_bf16 && dW && workspace, "%s: null pointer", who);
+    // the TMA reduce-add, the split-K partial tiles and splitk_reduce_kernel all move float4s
+    PIVP_REQUIRE(!(reinterpret_cast<uintptr_t>(dW) & 15) && !(reinterpret_cast<uintptr_t>(workspace) & 15),
+                 "%s: dW and workspace must be 16-byte aligned", who);
     PIVP_REQUIRE(ntaps >= 1 && ntaps <= 25, "%s: 1..25 taps", who);
     PIVP_REQUIRE(Cx >= 16 && Cx <= 256 && Cx % 16 == 0 && N4 >= 8 && N4 % 8 == 0 && dg_cs >= N4 && dg_cs % 8 == 0,
                  "%s: Cx must be a multiple of 16 <= 256, N4 a multiple of 8, rows 16-byte aligned", who);
@@ -382,10 +385,10 @@ static int launch_wgrad(const void* dg_bf16, int dg_cs, const void* xh_bf16, int
     if (bst > 8) bst = 8;
     if (bst < 2) bst = 2;
     g.b_stages = bst;
-    // dW reachable by TMA and two staging buffers fit the (dead) operand rings: reduce-add the partial tiles into dW, no workspace, no reduce launch
+    // whole 32-channel boxes and two staging buffers fit the (dead) operand rings: reduce-add the partial tiles into dW, no workspace, no reduce launch
     static const int tma_env = getenv("PIVP_TC_WGRAD_TMA") ? atoi(getenv("PIVP_TC_WGRAD_TMA")) : 1;
     const size_t ring_bytes = (size_t)WG_ASTAGES * 16384 + (size_t)bst * chunks * 8192;
-    g.tma_out = tma_env && Cx % 32 == 0 && !(reinterpret_cast<uintptr_t>(dW) & 15) && 2 * (size_t)(Cx / 32) * 16384 <= ring_bytes;
+    g.tma_out = tma_env && Cx % 32 == 0 && 2 * (size_t)(Cx / 32) * 16384 <= ring_bytes;
     CUtensorMap map_o;
     memset(&map_o, 0, sizeof(map_o));
     if (g.tma_out) {
@@ -432,6 +435,8 @@ int pivp_tc_wgrad5x5(const void* dg_bf16, const void* xh_bf16, int xh_cs, int SB
     PIVP_REQUIRE(N4 % 128 == 0 && xh_cs >= (Cx + 63) / 64 * 64, "tc_wgrad5x5: 4C must be a multiple of 128 and XH rows hold ceil(Cx/64)*64 channels");
     if (wgrad_halo_supported(H, W, Cx, N4)) {
         PIVP_REQUIRE(dg_bf16 && xh_bf16 && dW && workspace, "tc_wgrad5x5: null pointer");
+        PIVP_REQUIRE(!(reinterpret_cast<uintptr_t>(dW) & 15) && !(reinterpret_cast<uintptr_t>(workspace) & 15),
+                     "tc_wgrad5x5: dW and workspace must be 16-byte aligned");
         const int splits = launch_wgrad5x5_halo(dg_bf16, N4, xh_bf16, xh_cs, SB, H, W, Cx, N4, (float*)workspace, ws_bytes, dW, stream, "tc_wgrad5x5");
         if (splits <= 0) return splits;                // 0: the kernel added its partial tiles into dW itself (TMA reduce-add)
         const long n = (long)N4 * 25 * Cx, stride = (long)((N4 + 127) / 128 * 128) * 25 * Cx;

@@ -251,9 +251,9 @@ int launch_wgrad5x5_halo(const void* dg_bf16, int dg_cs, const void* xh_bf16, in
     Geom g;
     int splits;
     plan(Cx, N4, H, W, SB, &g, &splits);
-    // dW reachable by TMA (16-byte aligned, whole 32-channel boxes): the partial tiles are reduce-added into it directly, 0 splits returned
+    // whole 32-channel boxes (dW is 16-byte aligned, pivp_tc_wgrad5x5 checks it): the partial tiles are reduce-added into dW directly, 0 splits returned
     static const int tma_env = getenv("PIVP_TC_WGRAD_TMA") ? atoi(getenv("PIVP_TC_WGRAD_TMA")) : 1;
-    g.tma_out = tma_env && dW && Cx % 32 == 0 && !(reinterpret_cast<uintptr_t>(dW) & 15);
+    g.tma_out = tma_env && Cx % 32 == 0;
     CUtensorMap map_o;
     memset(&map_o, 0, sizeof(map_o));
     if (g.tma_out) {
