@@ -195,12 +195,32 @@ int pivp_stp_fused_bwd(const float* g_out, const float* prev, const float* enc7_
  *      CDNA  L = num_masks + 1: sigmoid(relu(enc7_pre)) (:315-317), then the num_masks per-sample cross-correlations (:326-347)
  *      DNA   L = 1: the 25-tap per-pixel transform with the truncated windows of :395-405
  *      STP   L = num_masks: sigmoid(enc7_pre) (:454-455), then num_masks - 1 samplings with the one shared theta (:465-470)
- *      Forward only; training goes through the fused entry points above. */
+ *      Model itself trains through the fused entry points above; the backward below serves a link called in its reference form. */
 int pivp_cdna_transform(const float* prev, const float* enc7_pre, const float* kern_raw, float* out, int B, int H, int W, int num_masks,
                         void* stream);
 int pivp_dna_transform(const float* prev, const float* enc7_pre, float* out, int B, int H, int W, void* stream);
 int pivp_stp_transform(const float* prev, const float* enc7_pre, const float* theta_raw, float* out, int B, int H, int W, int num_masks,
                        int oob_border, void* stream);
+/* Backward of the three lists.  g_list = HOST array of L device pointers (L as above), entry i = the gradient of list entry i,
+ * (B,3,H,W) contiguous, or NULL when that entry has no gradient (it is not read; e.g. the last CDNA entry, which the reference
+ * composite's zip(transformed, mask_list[1:]) never uses).  g_list itself must not be NULL.  g_enc7 = gradient of the returned enc7
+ * (relu(enc7_pre) for CDNA / DNA, enc7_pre for STP), may be NULL.
+ *  - d_enc7_pre, d_kern_raw (B,25*num_masks), d_theta_raw (B,6) are OVERWRITTEN.
+ *  - d_prev (optional, NULL = not computed) is overwritten, or added to when accumulate_dprev != 0.  DNA has none: its taps are
+ *    detached (:404).  STP with no live sampled entry (L = 1, or all of entries 1 .. L-1 NULL) only zeroes d_prev (if not accumulating).
+ *  - 1 <= num_masks <= 64.  d_kern_raw, d_theta_raw and the CDNA d_prev are deterministic (per-band partials in `workspace`, no float
+ *    atomics); the STP d_prev is a scatter-add.  CDNA / DNA stage bands of the image in 48 KB of shared memory: wider images than that
+ *    allows (CDNA W > 345 at num_masks = 64, DNA W > 815) are PIVP_EINVAL. */
+size_t pivp_cdna_transform_bwd_workspace_bytes(int B, int H, int W, int num_masks);
+int pivp_cdna_transform_bwd(const float* const* g_list, const float* g_enc7, const float* prev, const float* enc7_pre, const float* kern_raw,
+                            float* d_enc7_pre, float* d_kern_raw, float* d_prev, int accumulate_dprev,
+                            int B, int H, int W, int num_masks, void* workspace, size_t ws_bytes, void* stream);
+int pivp_dna_transform_bwd(const float* const* g_list, const float* g_enc7, const float* prev, const float* enc7_pre, float* d_enc7_pre,
+                           int B, int H, int W, void* stream);
+size_t pivp_stp_transform_bwd_workspace_bytes(int B, int H, int W, int num_masks);
+int pivp_stp_transform_bwd(const float* const* g_list, const float* g_enc7, const float* prev, const float* enc7_pre, const float* theta_raw,
+                           float* d_enc7_pre, float* d_theta_raw, float* d_prev, int accumulate_dprev,
+                           int B, int H, int W, int num_masks, int oob_border, void* workspace, size_t ws_bytes, void* stream);
 
 /* ---- inference preprocessing (predict_model.py:118-123): F.resize_images (bilinear, positions linspace(0, W-1, OW) in float64, corner
  *      indices clipped to [0, W-2]) fused with the cast and the division: y = resize(x) / scale (divide != 0) or * scale.

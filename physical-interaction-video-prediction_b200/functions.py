@@ -5,6 +5,8 @@ shape -- ``forward(inputs) -> outputs`` and ``backward(inputs, grad_outputs) -> 
 INTEGRATION.md's Chainer adapter is a three-line subclass.  Inputs are fp32, contiguous, NCHW like the
 reference's Variables.  No arithmetic happens in torch: it only owns the memory and the stream.
 """
+import ctypes
+
 import numpy as np
 import torch
 
@@ -112,6 +114,110 @@ class STPCompositeFunction(object):
         L.call("pivp_stp_fused_bwd", _p(g), _p(prev), _p(e), _p(a), _p(th), _p(de), _p(da), _p(dth), _p(dp),
                B, H, W, self.M, self.oob, _p(ws), nb, _s(prev))
         return dp, de, da, dth
+
+
+def _glist(grads):
+    """Chainer-style grad_outputs of a list (None = no gradient) -> host array of device pointers (None -> NULL)."""
+    _chk(*grads)
+    return (ctypes.c_void_p * len(grads))(*[_p(g) for g in grads])
+
+
+def _relu_out(e):
+    """relu(e) through the library's mask kernel: the reference's returned enc7 (ref:315, 388)."""
+    out = e.clone()
+    lib().call("pivp_relu_mask", _p(e), _p(out), out.numel(), _s(e))
+    return out
+
+
+class CDNATransformFunction(object):
+    """The reference call form of StatelessCDNA (train_model.py:315-347): transform list + enc7, un-fused.
+
+    inputs: prev (B,3,H,W), enc7_pre (B,3,H,W), kern_raw (B,25*M).  outputs: the M+1 list entries (B,3,H,W) -- sigmoid(relu(enc7_pre)),
+    then prev cross-correlated with each normalised kernel -- followed by enc7 = relu(enc7_pre).  backward takes the M+2 output gradients
+    (None allowed) and returns the gradients of (prev, enc7_pre, kern_raw)."""
+
+    def __init__(self, num_masks):
+        self.M = int(num_masks)
+
+    def forward(self, inputs):
+        prev, e, k = inputs
+        _chk(prev, e, k)
+        B, _, H, W = prev.shape
+        out = torch.empty(self.M + 1, B, 3, H, W, dtype=torch.float32, device=prev.device)
+        lib().call("pivp_cdna_transform", _p(prev), _p(e), _p(k), _p(out), B, H, W, self.M, _s(prev))
+        return tuple(out[i] for i in range(self.M + 1)) + (_relu_out(e),)
+
+    def backward(self, inputs, grad_outputs, need_dprev=True):
+        prev, e, k = inputs
+        _chk(prev, e, k)
+        B, _, H, W = prev.shape
+        gl = _glist(grad_outputs[:self.M + 1])
+        ge = grad_outputs[self.M + 1]
+        _chk(ge)
+        L = lib()
+        nb = L.query("pivp_cdna_transform_bwd_workspace_bytes", B, H, W, self.M)
+        ws = torch.empty(nb, dtype=torch.uint8, device=prev.device)
+        de, dk = torch.empty_like(e), torch.empty_like(k)
+        dp = torch.empty_like(prev) if need_dprev else None
+        L.call("pivp_cdna_transform_bwd", gl, _p(ge), _p(prev), _p(e), _p(k), _p(de), _p(dk), _p(dp), 0, B, H, W, self.M, _p(ws), nb, _s(prev))
+        return dp, de, dk
+
+
+class DNATransformFunction(object):
+    """The reference call form of StatelessDNA (train_model.py:388-414).  inputs: prev, enc7_pre (B,25,H,W); outputs: the one
+    transformed image and enc7 = relu(enc7_pre).  The taps are detached in the reference (:404), so the gradient of prev is None."""
+
+    def forward(self, inputs):
+        prev, e = inputs
+        _chk(prev, e)
+        B, _, H, W = prev.shape
+        out = torch.empty_like(prev)
+        lib().call("pivp_dna_transform", _p(prev), _p(e), _p(out), B, H, W, _s(prev))
+        return out, _relu_out(e)
+
+    def backward(self, inputs, grad_outputs):
+        prev, e = inputs
+        _chk(prev, e)
+        B, _, H, W = prev.shape
+        gl = _glist(grad_outputs[:1])
+        ge = grad_outputs[1]
+        _chk(ge)
+        de = torch.empty_like(e)
+        lib().call("pivp_dna_transform_bwd", gl, _p(ge), _p(prev), _p(e), _p(de), B, H, W, _s(prev))
+        return None, de
+
+
+class STPTransformFunction(object):
+    """The reference call form of StatelessSTP (train_model.py:454-470).  inputs: prev, enc7_pre (B,3,H,W), theta_raw (B,6) (the shared
+    Linear output before the identity is added); outputs: the num_masks list entries -- sigmoid(enc7_pre), then num_masks - 1 samplings
+    with the one theta -- followed by enc7 = enc7_pre.  backward returns the gradients of (prev, enc7_pre, theta_raw)."""
+
+    def __init__(self, num_masks, oob="zeros"):
+        self.M, self.oob = int(num_masks), 1 if oob == "border" else 0
+
+    def forward(self, inputs):
+        prev, e, th = inputs
+        _chk(prev, e, th)
+        B, _, H, W = prev.shape
+        out = torch.empty(self.M, B, 3, H, W, dtype=torch.float32, device=prev.device)
+        lib().call("pivp_stp_transform", _p(prev), _p(e), _p(th), _p(out), B, H, W, self.M, self.oob, _s(prev))
+        return tuple(out[i] for i in range(self.M)) + (e,)
+
+    def backward(self, inputs, grad_outputs, need_dprev=True):
+        prev, e, th = inputs
+        _chk(prev, e, th)
+        B, _, H, W = prev.shape
+        gl = _glist(grad_outputs[:self.M])
+        ge = grad_outputs[self.M]
+        _chk(ge)
+        L = lib()
+        nb = L.query("pivp_stp_transform_bwd_workspace_bytes", B, H, W, self.M)
+        ws = torch.empty(nb, dtype=torch.uint8, device=prev.device)
+        de, dth = torch.empty_like(e), torch.empty_like(th)
+        dp = torch.empty_like(prev) if need_dprev else None
+        L.call("pivp_stp_transform_bwd", gl, _p(ge), _p(prev), _p(e), _p(th), _p(de), _p(dth), _p(dp), 0, B, H, W, self.M, self.oob,
+               _p(ws), nb, _s(prev))
+        return dp, de, dth
 
 
 def nchw_to_nhwc(x):

@@ -150,6 +150,7 @@ class _Stateless(object):
         ``identity_params`` Linear) in Chainer layout as attributes ``<name>_W`` / ``<name>_b``, created lazily with Chainer's default
         initialisers like ``L.Linear(in_size=None)``, or set by the caller (``load(params, prefix="model/")`` takes a checkpoint dict).
         ``transformed_list`` is the un-fused list Model.__call__ composites at ref:725-728.
+        ``link.backward(g_transformed, g_enc7=None)`` is its backward, for a link dropped into the reference Model.
       * the FUSED form ``link.fused(prev_image, enc7_pre, mask_pre, ...) -> gen_image``: transform + mask softmax + composite in one
         kernel, which is what ``Model`` runs (the list never reaches memory).  A call with the fused arity is routed there.
     """
@@ -179,7 +180,8 @@ class _Stateless(object):
         B, C, H, W = enc6.shape
         Wt = self._param("enc7_W", (C, self.NE, 1, 1), enc6.device, fan_in=self.NE)
         b = self._param("enc7_b", (self.NE,), enc6.device)
-        return Fn.Deconvolution2DFunction(1, 0, (H, W)).forward((enc6.contiguous(), Wt, b))[0]
+        self._enc6 = enc6.contiguous()                                                  # kept for backward()
+        return Fn.Deconvolution2DFunction(1, 0, (H, W)).forward((self._enc6, Wt, b))[0]
 
     def _linear(self, name, x, out_size, relu=0):
         B, K = x.shape
@@ -189,6 +191,36 @@ class _Stateless(object):
         lib().call("pivp_linear_fwd", x.data_ptr(), K, Wt.data_ptr(), b.data_ptr(), y.data_ptr(), B, K, out_size, relu,
                    torch.cuda.current_stream(x.device).cuda_stream)
         return y
+
+    def _linear_bwd(self, name, x, dy):
+        """Backward of ``_linear`` (without its ReLU): returns dx, puts dW / db into ``self.grads``."""
+        Wt = getattr(self, name + "_W")
+        B, K = x.shape
+        N = Wt.shape[0]
+        dx = torch.empty_like(x)
+        dW, db = torch.zeros_like(Wt), torch.zeros(N, dtype=torch.float32, device=x.device)      # accumulated into
+        lib().call("pivp_linear_bwd", dy.data_ptr(), x.data_ptr(), K, Wt.data_ptr(), dx.data_ptr(), K, 0, dW.data_ptr(), db.data_ptr(),
+                   B, K, N, torch.cuda.current_stream(x.device).cuda_stream)
+        self.grads["model/%s/W" % name], self.grads["model/%s/b" % name] = dW, db
+        return dx
+
+    def backward(self, g_transformed, g_enc7=None):
+        """Backward of the reference call form.  ``g_transformed``: the gradients of the returned list, one per entry, ``None`` for an
+        entry without one (the reference Model composites with ``zip(transformed, mask_list[1:])``, ref:725-728, so the last CDNA entry
+        never gets one); ``g_enc7``: that of the returned enc7, or ``None``.  Returns ``(g_enc6, g_hidden5, g_prev)`` shaped like
+        ``encs[6]``, ``hiddens[4]`` and ``prev_image`` (``None`` where the link has no path: DNA's hidden5, and its prev_image, whose taps
+        the reference detaches, ref:404).  The parameter gradients go to ``self.grads`` in Chainer layout, keyed as ``load()`` reads them
+        (``model/enc7/W`` ...)."""
+        g_list = tuple(None if g is None else g.contiguous() for g in g_transformed)
+        if len(g_list) != self._nlist:
+            raise ValueError("expected %d list gradients, got %d" % (self._nlist, len(g_list)))
+        g_enc7 = None if g_enc7 is None else g_enc7.contiguous()
+        self.grads = {}
+        g_e7pre, g_hidden5, g_prev = self._transform_bwd(g_list, g_enc7)
+        H, W = self._enc6.shape[2:]
+        g_enc6, dW, db = Fn.Deconvolution2DFunction(1, 0, (H, W)).backward((self._enc6, self.enc7_W, self.enc7_b), (g_e7pre,))
+        self.grads["model/enc7/W"], self.grads["model/enc7/b"] = dW, db
+        return g_enc6, g_hidden5, g_prev
 
 
 class StatelessCDNA(_Stateless):
@@ -212,7 +244,14 @@ class StatelessCDNA(_Stateless):
         lib().call("pivp_cdna_transform", prev_image.contiguous().data_ptr(), enc7_pre.data_ptr(), kern_raw.data_ptr(), out.data_ptr(), B, H, W,
                    self.num_masks, torch.cuda.current_stream(out.device).cuda_stream)
         self.enc7_pre, self.kern_raw = enc7_pre, kern_raw
+        self._prev, self._h5, self._h5_shape = prev_image.contiguous(), hiddens[4].reshape(int(batch_size), -1).contiguous(), hiddens[4].shape
+        self._nlist = self.num_masks + 1
         return [out[i] for i in range(self.num_masks + 1)], enc7_pre.clamp(min=0)          # ref:315 enc7 = relu(enc7)
+
+    def _transform_bwd(self, g_list, g_enc7):
+        g_prev, g_e, g_k = Fn.CDNATransformFunction(self.num_masks).backward((self._prev, self.enc7_pre, self.kern_raw), g_list + (g_enc7,))
+        g_h5 = self._linear_bwd("cdna_kerns", self._h5, g_k)
+        return g_e, g_h5.reshape(self._h5_shape), g_prev
 
 
 class StatelessDNA(_Stateless):
@@ -236,7 +275,12 @@ class StatelessDNA(_Stateless):
         lib().call("pivp_dna_transform", prev_image.contiguous().data_ptr(), enc7_pre.data_ptr(), out.data_ptr(), B, H, W,
                    torch.cuda.current_stream(out.device).cuda_stream)
         self.enc7_pre = enc7_pre
+        self._prev, self._nlist = prev_image.contiguous(), 1
         return [out[0]], enc7_pre.clamp(min=0)
+
+    def _transform_bwd(self, g_list, g_enc7):
+        _, g_e = Fn.DNATransformFunction().backward((self._prev, self.enc7_pre), g_list + (g_enc7,))
+        return g_e, None, None
 
 
 class StatelessSTP(_Stateless):
@@ -262,7 +306,18 @@ class StatelessSTP(_Stateless):
         lib().call("pivp_stp_transform", prev_image.contiguous().data_ptr(), enc7.data_ptr(), theta_raw.data_ptr(), out.data_ptr(), B, H, W,
                    n, 1 if kw.get("oob", "zeros") == "border" else 0, torch.cuda.current_stream(out.device).cuda_stream)
         self.enc7_pre, self.theta_raw = enc7, theta_raw
+        self._prev, self._h5, self._h5_shape = prev_image.contiguous(), hiddens[4].reshape(int(batch_size), -1).contiguous(), hiddens[4].shape
+        self._s, self._nlist, self._oob = s_, n, kw.get("oob", "zeros")
         return [out[i] for i in range(n)], enc7
+
+    def _transform_bwd(self, g_list, g_enc7):
+        f = Fn.STPTransformFunction(self._nlist, self._oob)
+        g_prev, g_e, g_th = f.backward((self._prev, self.enc7_pre, self.theta_raw), g_list + (g_enc7,))
+        g_s = self._linear_bwd("identity_params", self._s, g_th)
+        lib().call("pivp_relu_mask", self._s.data_ptr(), g_s.data_ptr(), g_s.numel(),       # the ReLU between the two Linears (ref:457)
+                   torch.cuda.current_stream(g_s.device).cuda_stream)
+        g_h5 = self._linear_bwd("stp_input", self._h5, g_s)
+        return g_e, g_h5.reshape(self._h5_shape), g_prev
 
 
 # ----------------------------------------------------------------------------- Model
