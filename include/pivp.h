@@ -59,7 +59,9 @@ int pivp_conv2d_wgrad(const float* x, int x_cs, int x_co, int B, int H, int W, i
 int pivp_colsum(const float* v, int v_cs, int v_co, int P, int N, float* out, void* stream);
 
 /* ---- BasicConvLSTMCell gate math (train_model.py:269-272; D.5) ---------------------------------------- */
-/* gates: (M, 4C) pre-activations in, activated gates out (saved for backward). c_prev may be NULL (zeros). */
+/* gates: (M, 4C) pre-activations in, activated gates out (saved for backward). c_prev may be NULL (zeros).
+ * c_prev == c_out is allowed (the cell state updated in place): every element of c_prev is read once, by the thread that then writes
+ * the same element of c_out, before it writes it. */
 int pivp_lstm_gates_fwd(float* gates, const float* c_prev, float* c_out, float* h_out, int h_cs, int h_co,
                         void* h_bf16, int hb_cs, int hb_co, long M, int C, float forget_bias, void* stream);
 /* dh = dh_a (dense, may be NULL) + dh_b (view, may be NULL); dc in/out (dc_valid=0: treat incoming dc as 0);
@@ -164,7 +166,9 @@ int pivp_heads_fwd(const float* x, int x_cs, int x_co, const float* W, const flo
                    int B, int HW, void* stream);
 /* forward on relu(LayerNorm(x)) in one launch (norm_enc6 + ReLU `:601, 698` then the heads): x = the LayerNorm input, partial = the
  * [B][HW*64/4096] (mean, M2) pairs written by pivp_tc_conv_taps_multi_ln, y = normalised rows kept for the backward, stats [B][2] =
- * (mean, rstd) for pivp_layernorm_bwd.  HW must be a multiple of 128. */
+ * (mean, rstd) for pivp_layernorm_bwd.  HW must be a multiple of 128.
+ * y == NULL: the normalised rows are not written (forward-only prediction; a kernel instantiation without that store).  stats stays
+ * required. */
 int pivp_heads_fwd_ln(const float* x, int x_cs, int x_co, const float* gamma, const float* beta, const float* partial, float eps, float* stats,
                       float* y, int y_cs, int y_co, const float* W, const float* bias, float* out_a, int Na, float* out_b, int NH,
                       int B, int HW, void* stream);
@@ -242,7 +246,13 @@ int pivp_tc_set_debug_buffer(void* device_buffer);
  *         ln_partial (optional, mode 1 on maps with H % 16 == 0, W % 8 == 0): the epilogue also writes the LayerNorm statistics of h as
  *         per-tile (mean, M2) pairs in the workspace layout of pivp_layernorm_fwd, which can then be called with relu | 2 (skip its
  *         own statistics pass).
- *         flags: bit 0 = accurate tanhf/expf instead of tanh.approx; bit 1 = `gates` points to bf16 storage (M,4C) (pivp_lstm_gates_bwd_bf16).
+ *         flags: bit 0 = accurate tanhf/expf instead of tanh.approx; bit 1 = `gates` points to bf16 storage (M,4C) (pivp_lstm_gates_bwd_bf16);
+ *         bit 2 = no gate storage: the activated gates are not written (forward-only prediction: only the backward pass reads them) and
+ *         `gates` may be NULL.  Chosen at compile time (a kernel instantiation without the gate store).  Bit 2 without mode 1, or a NULL
+ *         `gates` without bit 2, returns PIVP_EINVAL before any CUDA call.
+ *         c_prev == c_out is allowed in every epilogue variant (cell state updated in place): each c_prev element is read by the thread that
+ *         computes c_t for the same pixel and channel, before the accumulator wait (halo kernel) or before its own store (per-tap kernel),
+ *         and written only after that read.
  * Returns PIVP_EUNSUPPORTED when B*H*W cannot be cut into 128-pixel TMA boxes. */
 int pivp_tc_conv5x5(const void* in_bf16, int in_cs, int B, int H, int W, int Kc,
                     const void* wt_bf16, int N, int BN,
@@ -258,7 +268,8 @@ int pivp_tc_conv5x5(const void* in_bf16, int in_cs, int B, int H, int W, int Kc,
  * written, then every thread normalises the h values it still holds in registers: y = (h - mean) * rstd * gamma + beta -> fp32 view `y`
  * (+ optional bf16 view), stats[b] = (mean, rstd) for the LayerNorm backward.  gamma / beta in the sample's H*W*C order.
  * counter: B unsigned ints owned by this layer, zeroed once (never reset: every launch adds the same number of arrivals per sample).
- * Needs the halo-patch geometry (H % 16 == 0, W % 8 == 0), H*W*C % 4096 == 0 and at most 148 CTAs (all resident at once). */
+ * Needs the halo-patch geometry (H % 16 == 0, W % 8 == 0), H*W*C % 4096 == 0 and at most 148 CTAs (all resident at once).
+ * Always stores the gates: flags bit 2 is PIVP_EINVAL here. */
 int pivp_tc_conv5x5_ln(const void* in_bf16, int in_cs, int B, int H, int W, int Kc, const void* wt_bf16, int C, const float* bias,
                        void* gates_bf16, const float* c_prev, float* c_out, float* h_out, int h_cs, int h_co, void* h_bf16, int hb_cs, int hb_co,
                        float forget_bias, int flags, float* ln_partial,

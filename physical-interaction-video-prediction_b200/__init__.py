@@ -9,7 +9,8 @@ from . import layout                                                      # noqa
 
 def __getattr__(name):
     # torch-dependent modules are imported lazily so that `import pivp_b200` works in a build-only environment
-    if name in ("functions", "links", "engine", "tensorcore", "parallel", "train", "data", "serializers", "rollout", "train_loop"):
+    if name in ("functions", "links", "engine", "tensorcore", "parallel", "train", "data", "serializers", "rollout", "train_loop",
+                "predictor"):
         import importlib
         return importlib.import_module("." + name, __name__)
     if name in ("Model", "Adam", "BasicConvLSTMCell", "LayerNormalizationConv2D", "StatelessCDNA", "StatelessDNA",
@@ -23,6 +24,9 @@ def __getattr__(name):
     if name in ("Rollout", "predict"):
         from . import rollout
         return getattr(rollout, name)
+    if name == "Predictor":
+        from .predictor import Predictor
+        return Predictor
     if name in ("save_npz", "load_npz"):
         from . import serializers
         return getattr(serializers, name)

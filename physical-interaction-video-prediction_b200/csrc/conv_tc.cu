@@ -54,6 +54,8 @@ struct TcGeomPack {
                      // accumulator of BN columns per phase (grid z = 1) -- a quarter of the CTAs, so a 64x64 deconvolution is ONE wave
 };
 
+// GATES = false: mode 1 without the gate store (pivp_tc_conv5x5 flags bit 2, ep.gates == null)
+template <bool GATES>
 __global__ void __launch_bounds__(TC_THREADS, 2)
 conv_taps_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ TcMapsB maps_b, const __grid_constant__ TcMapsOut maps_o,
                     const __grid_constant__ TcMapsOut maps_ob, const __grid_constant__ TcGeomPack gp, TcEpilogue ep) {
@@ -216,7 +218,7 @@ conv_taps_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                         make_float2(0.5f * (mab + mce), (sab + sce) + dd * dd * 1024.f);
                 }
             } else if (!gp.out_bytes) {
-                tc_epilogue_row(ep, trow + (uint32_t)(p * g.BN), m, orow, n0, g.BN, n_tile, bias_s);
+                tc_epilogue_row<GATES>(ep, trow + (uint32_t)(p * g.BN), m, orow, n0, g.BN, n_tile, bias_s);
             }
         }
         tc_fence_before();
@@ -382,12 +384,14 @@ static int launch_conv_taps_multi(const void* in_bf16, int in_cs, int B, int H, 
     const size_t smem = 1024 + (size_t)out_bytes + (size_t)stages * stage_bytes + (2 * stages + TC_MAXPH) * 8 + 16 + (size_t)BN * 4 + TC_MAXPH * 32 * sizeof(float2);
     static PerDeviceOnce attr_once;            // the opt-in is per device
     if (attr_once.need()) {
-        cudaError_t e = cudaFuncSetAttribute(conv_taps_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        cudaError_t e = cudaFuncSetAttribute(conv_taps_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_taps_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         if (e != cudaSuccess) { set_error("%s: cudaFuncSetAttribute: %s", who, cudaGetErrorString(e)); return PIVP_ECUDA; }
     }
     const long M = (long)B * H * W;
     dim3 grid((unsigned)(M / TC_BM), (unsigned)(N / BN), (unsigned)(fuse_ph ? 1 : nph));
-    launch_k(conv_taps_tc_kernel, grid, dim3(TC_THREADS), smem, stream, map_a, mb, mo, mob, gp, ep);
+    if (ep.mode == 1 && !ep.gates) launch_k(conv_taps_tc_kernel<false>, grid, dim3(TC_THREADS), smem, stream, map_a, mb, mo, mob, gp, ep);
+    else launch_k(conv_taps_tc_kernel<true>, grid, dim3(TC_THREADS), smem, stream, map_a, mb, mo, mob, gp, ep);
     return check_launch(who);
 }
 
@@ -443,8 +447,11 @@ static int tc_conv5x5_impl(const void* in_bf16, int in_cs, int B, int H, int W, 
                     void* h_t, long h_t_ld, int hT_co,
                     int C, float forget_bias, int flags, float* ln_partial, const LnFuse& lf, void* stream) {
     PIVP_REQUIRE(in_cs >= Kc, "tc_conv5x5: row stride smaller than Kc");
+    const bool no_gates = (flags >> 2) & 1;       // forward-only: the activated gates are not stored (nothing reads them without a backward pass)
+    PIVP_REQUIRE(!no_gates || mode == 1, "tc_conv5x5: flags bit 2 (no gate storage) needs mode 1");
     if (mode == 1) {
-        PIVP_REQUIRE(BN == 128 && N == 4 * C && C % 32 == 0 && gates && c_out && h_out && bias, "tc_conv5x5: gate epilogue needs BN=128, N=4C, bias");
+        PIVP_REQUIRE(BN == 128 && N == 4 * C && C % 32 == 0 && (gates || no_gates) && c_out && h_out && bias,
+                     "tc_conv5x5: gate epilogue needs BN=128, N=4C, bias, and gates unless flags bit 2 is set");
         PIVP_REQUIRE(h_cs % 4 == 0 && h_co % 4 == 0 && (!h_bf16 || (hb_cs % 8 == 0 && hb_co % 8 == 0)), "tc_conv5x5: h views must be 16-byte aligned");
     } else {
         PIVP_REQUIRE(mode == 0 && out && out_cs % 4 == 0 && out_co % 4 == 0, "tc_conv5x5: plain epilogue needs a 16-byte aligned fp32 view");
@@ -453,7 +460,7 @@ static int tc_conv5x5_impl(const void* in_bf16, int in_cs, int B, int H, int W, 
     for (int t = 0; t < 25; ++t) { dy[t] = t / 5 - 2; dx[t] = t % 5 - 2; co[t] = 0; }
     TcEpilogue ep;
     memset(&ep, 0, sizeof(ep));
-    ep.mode = mode; ep.bias = bias; ep.out = out; ep.out_cs = out_cs; ep.out_co = out_co; ep.gates = gates; ep.c_prev = c_prev;
+    ep.mode = mode; ep.bias = bias; ep.out = out; ep.out_cs = out_cs; ep.out_co = out_co; ep.gates = no_gates ? nullptr : gates; ep.c_prev = c_prev;
     ep.c_out = c_out; ep.h_out = h_out; ep.h_cs = h_cs; ep.h_co = h_co; ep.h_bf16 = (__nv_bfloat16*)h_bf16; ep.hb_cs = hb_cs; ep.hb_co = hb_co;
     ep.h_t = (__nv_bfloat16*)h_t; ep.h_t_ld = h_t_ld; ep.hT_co = hT_co;
     ep.C = C; ep.forget_bias = forget_bias; ep.accurate = flags & 1; ep.gates_bf16 = (flags >> 1) & 1;
@@ -500,6 +507,7 @@ int pivp_tc_conv5x5_ln(const void* in_bf16, int in_cs, int B, int H, int W, int 
                        float* stats, void* counter, void* stream) {
     LnFuse lf{gamma, beta, y, y_cs, y_co, y_bf16, yb_cs, yb_co, stats, (unsigned*)counter, eps};
     PIVP_REQUIRE(gamma, "tc_conv5x5_ln: gamma is null");
+    PIVP_REQUIRE(!(flags & 4), "tc_conv5x5_ln: stores the gates always (flags bit 2 is for pivp_tc_conv5x5)");
     return tc_conv5x5_impl(in_bf16, in_cs, B, H, W, Kc, wt_bf16, 4 * C, 128, 1, bias, nullptr, 0, 0, (float*)gates_bf16, c_prev, c_out, h_out, h_cs, h_co,
                            h_bf16, hb_cs, hb_co, nullptr, 0, 0, C, forget_bias, flags | 2, ln_partial, lf, stream);
 }

@@ -75,7 +75,10 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t sbo_bytes
 // One CTA per SM: all shared memory that the MS patches leave goes to the weight ring, deep enough to cover the L2 round trip.
 // NP = patch buffers (compile-time: the buffer index and barrier parity of a block must stay on the uniform datapath, a run-time
 // modulus pushes the whole issue loop back onto vector registers + per-MMA R2UR / divergence checks).
-template <int MS, int NP>
+// GATES = false: the mode-1 epilogues store no activated gates (pivp_tc_conv5x5 flags bit 2: forward-only prediction, ep.gates == null).
+// c_prev may alias c_out in every mode-1 epilogue: a thread loads the c_prev elements of its own pixel row and channels before the
+// accumulator wait, and those elements are written (by a TMA store or the coalesced write-out) only after the barrier of the tile's warps.
+template <int MS, int NP, bool GATES>
 __global__ void __launch_bounds__(64 + 256 * MS, 1)
 conv5x5_halo_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, const __grid_constant__ OutMaps om,
                        Geom g, TcEpilogue ep) {
@@ -275,10 +278,12 @@ conv5x5_halo_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
                 for (int i = 0; i < 8; ++i) hv[cc + i] = hn[i];
                 const uint32_t k8 = (uint32_t)(c0 >> 3), k4 = (uint32_t)(c0 >> 2);       // 16-byte chunk of this thread's columns in a bf16 / fp32 row
                 uint4 pk;
-                pk = pack8_bf16(gj); st_shared_v4(sG + r128 + ((k8 ^ rsw) << 4), pk.x, pk.y, pk.z, pk.w);                       // box 0: j | i
-                pk = pack8_bf16(gi); st_shared_v4(sG + r128 + (((4u + k8) ^ rsw) << 4), pk.x, pk.y, pk.z, pk.w);
-                pk = pack8_bf16(gf); st_shared_v4(sG + 16384u + r128 + ((k8 ^ rsw) << 4), pk.x, pk.y, pk.z, pk.w);              // box 1: f | o
-                pk = pack8_bf16(go); st_shared_v4(sG + 16384u + r128 + (((4u + k8) ^ rsw) << 4), pk.x, pk.y, pk.z, pk.w);
+                if (GATES) {
+                    pk = pack8_bf16(gj); st_shared_v4(sG + r128 + ((k8 ^ rsw) << 4), pk.x, pk.y, pk.z, pk.w);                   // box 0: j | i
+                    pk = pack8_bf16(gi); st_shared_v4(sG + r128 + (((4u + k8) ^ rsw) << 4), pk.x, pk.y, pk.z, pk.w);
+                    pk = pack8_bf16(gf); st_shared_v4(sG + 16384u + r128 + ((k8 ^ rsw) << 4), pk.x, pk.y, pk.z, pk.w);          // box 1: f | o
+                    pk = pack8_bf16(go); st_shared_v4(sG + 16384u + r128 + (((4u + k8) ^ rsw) << 4), pk.x, pk.y, pk.z, pk.w);
+                }
                 st_shared_v4(sC + r128 + ((k4 ^ rsw) << 4), __float_as_uint(cn[0]), __float_as_uint(cn[1]), __float_as_uint(cn[2]), __float_as_uint(cn[3]));
                 st_shared_v4(sC + r128 + (((k4 + 1u) ^ rsw) << 4), __float_as_uint(cn[4]), __float_as_uint(cn[5]), __float_as_uint(cn[6]), __float_as_uint(cn[7]));
                 st_shared_v4(sH + r128 + ((k4 ^ rsw) << 4), __float_as_uint(hn[0]), __float_as_uint(hn[1]), __float_as_uint(hn[2]), __float_as_uint(hn[3]));
@@ -315,8 +320,10 @@ conv5x5_halo_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
             const int tiles_per_img = tiles_x * tiles_y;
             if (lw == 0) {
                 if (elect_one()) {
-                    tma_store_4d(&om.gates, sG, n0, oc1, oc2, oc3);
-                    tma_store_4d(&om.gates, sG + 16384u, n0 + 64, oc1, oc2, oc3);
+                    if (GATES) {
+                        tma_store_4d(&om.gates, sG, n0, oc1, oc2, oc3);
+                        tma_store_4d(&om.gates, sG + 16384u, n0 + 64, oc1, oc2, oc3);
+                    }
                     tma_store_4d(&om.c, sC, ch0, oc1, oc2, oc3);
                     tma_store_4d(&om.h, sH, ep.h_co + ch0, oc1, oc2, oc3);
                     tma_store_4d(&om.hb, sHB, ep.hb_co + ch0, oc1, oc2, oc3);
@@ -467,15 +474,17 @@ conv5x5_halo_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
                 tc_ld_wait();
                 if (ep.accurate) gate_math8<true>(gj, gi, gf, go, cp + cc, bias_s, c0, ep.forget_bias, cn, hn);
                 else gate_math8<false>(gj, gi, gf, go, cp + cc, bias_s, c0, ep.forget_bias, cn, hn);
-                float* gr = G + row * GP + c0;
-                *reinterpret_cast<float4*>(gr) = make_float4(gj[0], gj[1], gj[2], gj[3]);
-                *reinterpret_cast<float4*>(gr + 4) = make_float4(gj[4], gj[5], gj[6], gj[7]);
-                *reinterpret_cast<float4*>(gr + 32) = make_float4(gi[0], gi[1], gi[2], gi[3]);
-                *reinterpret_cast<float4*>(gr + 36) = make_float4(gi[4], gi[5], gi[6], gi[7]);
-                *reinterpret_cast<float4*>(gr + 64) = make_float4(gf[0], gf[1], gf[2], gf[3]);
-                *reinterpret_cast<float4*>(gr + 68) = make_float4(gf[4], gf[5], gf[6], gf[7]);
-                *reinterpret_cast<float4*>(gr + 96) = make_float4(go[0], go[1], go[2], go[3]);
-                *reinterpret_cast<float4*>(gr + 100) = make_float4(go[4], go[5], go[6], go[7]);
+                if (GATES) {
+                    float* gr = G + row * GP + c0;
+                    *reinterpret_cast<float4*>(gr) = make_float4(gj[0], gj[1], gj[2], gj[3]);
+                    *reinterpret_cast<float4*>(gr + 4) = make_float4(gj[4], gj[5], gj[6], gj[7]);
+                    *reinterpret_cast<float4*>(gr + 32) = make_float4(gi[0], gi[1], gi[2], gi[3]);
+                    *reinterpret_cast<float4*>(gr + 36) = make_float4(gi[4], gi[5], gi[6], gi[7]);
+                    *reinterpret_cast<float4*>(gr + 64) = make_float4(gf[0], gf[1], gf[2], gf[3]);
+                    *reinterpret_cast<float4*>(gr + 68) = make_float4(gf[4], gf[5], gf[6], gf[7]);
+                    *reinterpret_cast<float4*>(gr + 96) = make_float4(go[0], go[1], go[2], go[3]);
+                    *reinterpret_cast<float4*>(gr + 100) = make_float4(go[4], go[5], go[6], go[7]);
+                }
                 *reinterpret_cast<float4*>(Cc + row * CP + c0) = make_float4(cn[0], cn[1], cn[2], cn[3]);
                 *reinterpret_cast<float4*>(Cc + row * CP + c0 + 4) = make_float4(cn[4], cn[5], cn[6], cn[7]);
                 *reinterpret_cast<float4*>(Hh + row * CP + c0) = make_float4(hn[0], hn[1], hn[2], hn[3]);
@@ -517,7 +526,8 @@ conv5x5_halo_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
                     ep.ln_partial[(long)tb * ep.ln_S + (mt - tb * tiles_per_img) * (ep.C >> 5) + n_tile] = make_float2(mean, t2);
                 }
             }
-            if (ep.gates_bf16) {
+            if (!GATES) {
+            } else if (ep.gates_bf16) {
                 // bf16 gate storage: 256-byte rows, 16 lanes x 16 B per row, two rows per warp instruction
                 __nv_bfloat16* gb = reinterpret_cast<__nv_bfloat16*>(ep.gates);
                 const int sr = lane >> 4, l16 = lane & 15;
@@ -586,16 +596,16 @@ conv5x5_halo_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
     }
 }
 
-template <int MS, int NP>
+template <int MS, int NP, bool GATES>
 static int launch_ms_np(const CUtensorMap& map_a, const CUtensorMap& map_b, const OutMaps& om, const Geom& g, const TcEpilogue& ep, int tiles, int splits,
                         size_t smem, void* stream, const char* who) {
     static PerDeviceOnce attr_once;            // the opt-in is per device
     if (attr_once.need()) {
-        cudaError_t e = cudaFuncSetAttribute(conv5x5_halo_tc_kernel<MS, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaError_t e = cudaFuncSetAttribute(conv5x5_halo_tc_kernel<MS, NP, GATES>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         if (e != cudaSuccess) { set_error("%s(halo): cudaFuncSetAttribute: %s", who, cudaGetErrorString(e)); return PIVP_ECUDA; }
     }
     dim3 grid((unsigned)(tiles / MS), (unsigned)(g.N / g.BN), (unsigned)splits);
-    launch_k(conv5x5_halo_tc_kernel<MS, NP>, grid, dim3(64 + 256 * MS), smem, stream, map_a, map_b, om, g, ep);
+    launch_k(conv5x5_halo_tc_kernel<MS, NP, GATES>, grid, dim3(64 + 256 * MS), smem, stream, map_a, map_b, om, g, ep);
     return check_launch(who);
 }
 
@@ -648,9 +658,14 @@ static int launch_ms(const CUtensorMap& map_a, const CUtensorMap& map_b, const O
     // the fused LayerNorm's per-sample rendezvous needs every CTA of the launch resident at once: one CTA per SM, so at most 148 of them
     PIVP_REQUIRE(!ep.ln_gamma || (long)(tiles / MS) * (g.N / g.BN) * splits <= 148, "%s(halo): fused LayerNorm with more CTAs than SMs", who);
     PIVP_REQUIRE(ep.mode != 1 || g.tma_out || dead >= (size_t)MS * STG_FLOATS * 4 + 256, "%s(halo): operand ring too small to stage the gate epilogue", who);
-    if (MS == 1 && np == 3) return launch_ms_np<1, 3>(map_a, map_b, om, g, ep, tiles, splits, smem, stream, who);
-    if (MS == 1 && np == 2) return launch_ms_np<1, 2>(map_a, map_b, om, g, ep, tiles, splits, smem, stream, who);
-    return launch_ms_np<MS, 1>(map_a, map_b, om, g, ep, tiles, splits, smem, stream, who);
+    if (ep.mode == 1 && !ep.gates) {                    // forward-only: the instantiation without the gate store
+        if (MS == 1 && np == 3) return launch_ms_np<1, 3, false>(map_a, map_b, om, g, ep, tiles, splits, smem, stream, who);
+        if (MS == 1 && np == 2) return launch_ms_np<1, 2, false>(map_a, map_b, om, g, ep, tiles, splits, smem, stream, who);
+        return launch_ms_np<MS, 1, false>(map_a, map_b, om, g, ep, tiles, splits, smem, stream, who);
+    }
+    if (MS == 1 && np == 3) return launch_ms_np<1, 3, true>(map_a, map_b, om, g, ep, tiles, splits, smem, stream, who);
+    if (MS == 1 && np == 2) return launch_ms_np<1, 2, true>(map_a, map_b, om, g, ep, tiles, splits, smem, stream, who);
+    return launch_ms_np<MS, 1, true>(map_a, map_b, om, g, ep, tiles, splits, smem, stream, who);
 }
 
 }  // namespace halo
@@ -723,9 +738,10 @@ int launch_conv5x5_halo(const void* in_bf16, int in_cs, int B, int H, int W, int
             }
             return encode_tmap_ex(mp, dt, sw, base, 4, dims, str, box) == CUDA_SUCCESS;
         };
-        if (want && ep.mode == 1 && ep.gates_bf16 && ep.h_bf16 && !ep.h_t && a16(ep.gates) && a16(ep.c_out) && a16(ep.h_out) && a16(ep.h_bf16) &&
-            ep.C % 4 == 0 && ep.h_cs % 4 == 0 && ep.hb_cs % 8 == 0) {
-            g.tma_out = enc(&om.gates, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, CU_TENSOR_MAP_SWIZZLE_128B, ep.gates, 4 * ep.C, 2, 64) &&
+        // (no gate map without gate storage: forward-only launches, ep.gates == null)
+        if (want && ep.mode == 1 && (!ep.gates || (ep.gates_bf16 && a16(ep.gates))) && ep.h_bf16 && !ep.h_t && a16(ep.c_out) && a16(ep.h_out) &&
+            a16(ep.h_bf16) && ep.C % 4 == 0 && ep.h_cs % 4 == 0 && ep.hb_cs % 8 == 0) {
+            g.tma_out = (!ep.gates || enc(&om.gates, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, CU_TENSOR_MAP_SWIZZLE_128B, ep.gates, 4 * ep.C, 2, 64)) &&
                         enc(&om.c, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, CU_TENSOR_MAP_SWIZZLE_128B, ep.c_out, ep.C, 4, 32) &&
                         enc(&om.h, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, CU_TENSOR_MAP_SWIZZLE_128B, ep.h_out, ep.h_cs, 4, 32) &&
                         enc(&om.hb, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, CU_TENSOR_MAP_SWIZZLE_64B, ep.h_bf16, ep.hb_cs, 2, 32);

@@ -10,7 +10,9 @@ namespace pivp {
 // Gate buffer layout: row m holds 4*C values ordered [block of 32 channels][gate j,i,f,o][32 channels].
 __device__ __forceinline__ int gate_col(int ch, int gate) { return (ch >> 5) * 128 + gate * 32 + (ch & 31); }
 
-__global__ void lstm_gates_fwd_kernel(float* __restrict__ gates, const float* __restrict__ c_prev, float* __restrict__ c_out,
+// c_prev may alias c_out (the cell state updated in place): each thread reads c_prev[idx] once, before it writes c_out[idx], and no other
+// thread touches element idx -- hence no __restrict__ on those two.
+__global__ void lstm_gates_fwd_kernel(float* __restrict__ gates, const float* c_prev, float* c_out,
                                       View h_out, __nv_bfloat16* __restrict__ h_bf16, int hb_cs, int hb_co,
                                       long M, int C, float forget_bias) {
     pdl_enter();

@@ -80,7 +80,8 @@ __device__ __forceinline__ float2 ln_combine(const float2* __restrict__ partial,
     return make_float2(mu, 1.f / sqrtf(m2 / n + eps));
 }
 
-template <int BATCH>
+// Y = false: the normalised rows are not written (pivp_heads_fwd_ln with y == NULL: forward-only prediction, no backward reads them)
+template <int BATCH, bool Y>
 __device__ __forceinline__ void load_tile_ln(const float* __restrict__ x, int cs, int co, long m0, long M, float* xs, const LnIn& ln, float2 st,
                                              long e0) {
     constexpr int NL = TP * (C / 4) / TP;
@@ -106,12 +107,12 @@ __device__ __forceinline__ void load_tile_ln(const float* __restrict__ x, int cs
             o.z = fmaxf((v[k].z - st.x) * st.y * ga[k].z + be[k].z, 0.f);
             o.w = fmaxf((v[k].w - st.x) * st.y * ga[k].w + be[k].w, 0.f);
             *reinterpret_cast<float4*>(xs + r * XP + 4 * c4) = o;
-            if (m0 + r < M) *reinterpret_cast<float4*>(ln.y + (m0 + r) * ln.y_cs + ln.y_co + 4 * c4) = o;
+            if (Y && m0 + r < M) *reinterpret_cast<float4*>(ln.y + (m0 + r) * ln.y_cs + ln.y_co + 4 * c4) = o;
         }
     }
 }
 
-template <int NH>
+template <int NH, bool Y>
 __global__ void __launch_bounds__(TP) heads_fwd_kernel(const float* __restrict__ x, int cs, int co, const float* __restrict__ Wt,
                                                        const float* __restrict__ bias, float* __restrict__ out_a, int Na,
                                                        float* __restrict__ out_b, long M, int HW, LnIn ln) {
@@ -148,7 +149,7 @@ __global__ void __launch_bounds__(TP) heads_fwd_kernel(const float* __restrict__
     const long m0 = (long)blockIdx.x * TP;
     if (ln.gamma) {
         __syncthreads();                                         // st_s
-        load_tile_ln<8>(x, cs, co, m0, M, xs, ln, st_s, (m0 % HW) * C);
+        load_tile_ln<8, Y>(x, cs, co, m0, M, xs, ln, st_s, (m0 % HW) * C);
     } else {
         load_tile<16>(x, cs, co, m0, M, xs);
     }
@@ -320,8 +321,11 @@ static int heads_fwd_impl(const float* x, int x_cs, int x_co, const float* W, co
     PIVP_REQUIRE(hd::a16(x) && x_cs % 4 == 0 && x_co % 4 == 0, "heads_fwd: rows must be 16-byte aligned");
     const long M = (long)B * HW;
     const unsigned grid = (unsigned)((M + hd::TP - 1) / hd::TP);
-    if (NH == 14) launch_k(hd::heads_fwd_kernel<14>, dim3(grid), dim3(hd::TP), 0, (cudaStream_t)stream, x, x_cs, x_co, W, bias, out_a, Na, out_b, M, HW, ln);
-    else if (NH == 27) launch_k(hd::heads_fwd_kernel<27>, dim3(grid), dim3(hd::TP), 0, (cudaStream_t)stream, x, x_cs, x_co, W, bias, out_a, Na, out_b, M, HW, ln);
+    const bool y = !ln.gamma || ln.y;               // the LayerNorm form with y == NULL: the instantiation that does not write the normalised rows
+    if (NH == 14 && y) launch_k(hd::heads_fwd_kernel<14, true>, dim3(grid), dim3(hd::TP), 0, (cudaStream_t)stream, x, x_cs, x_co, W, bias, out_a, Na, out_b, M, HW, ln);
+    else if (NH == 27 && y) launch_k(hd::heads_fwd_kernel<27, true>, dim3(grid), dim3(hd::TP), 0, (cudaStream_t)stream, x, x_cs, x_co, W, bias, out_a, Na, out_b, M, HW, ln);
+    else if (NH == 14) launch_k(hd::heads_fwd_kernel<14, false>, dim3(grid), dim3(hd::TP), 0, (cudaStream_t)stream, x, x_cs, x_co, W, bias, out_a, Na, out_b, M, HW, ln);
+    else if (NH == 27) launch_k(hd::heads_fwd_kernel<27, false>, dim3(grid), dim3(hd::TP), 0, (cudaStream_t)stream, x, x_cs, x_co, W, bias, out_a, Na, out_b, M, HW, ln);
     else { set_error("heads_fwd: %d heads not instantiated (14 or 27)", NH); return PIVP_EUNSUPPORTED; }
     return check_launch("heads_fwd");
 }
@@ -335,14 +339,15 @@ int pivp_heads_fwd(const float* x, int x_cs, int x_co, const float* W, const flo
 
 /* The heads on relu(LayerNorm(x)) in ONE launch (norm_enc6 + ReLU, train_model.py:601, 698, then enc7 / masks): x = the LayerNorm INPUT (enc6's
  * deconvolution output), partial = the [B][HW*64/4096] (mean, M2) pairs the deconvolution's epilogue wrote (pivp_tc_conv_taps_multi_ln),
- * gamma / beta [HW*64]; y receives the normalised rows (the backward reads them), stats [B] the (mean, rstd) pairs pivp_layernorm_bwd needs.
+ * gamma / beta [HW*64]; y receives the normalised rows (the backward reads them; NULL: not written), stats [B] the (mean, rstd) pairs
+ * pivp_layernorm_bwd needs.
  * Replaces pivp_layernorm_fwd(relu | 2) + pivp_heads_fwd.  HW must be a multiple of 128 and HW*64 of 4096. */
 int pivp_heads_fwd_ln(const float* x, int x_cs, int x_co, const float* gamma, const float* beta, const float* partial, float eps, float* stats,
                       float* y, int y_cs, int y_co, const float* W, const float* bias, float* out_a, int Na, float* out_b, int NH,
                       int B, int HW, void* stream) {
-    PIVP_REQUIRE(gamma && beta && partial && stats && y, "heads_fwd_ln: null pointer");
+    PIVP_REQUIRE(gamma && beta && partial && stats, "heads_fwd_ln: null pointer");     // y may be NULL: the normalised rows are then not written
     PIVP_REQUIRE(HW % hd::TP == 0 && ((long)HW * hd::C) % 4096 == 0, "heads_fwd_ln: HW must be a multiple of 128");
-    PIVP_REQUIRE(hd::a16(gamma) && hd::a16(beta) && hd::a16(y) && y_cs % 4 == 0 && y_co % 4 == 0, "heads_fwd_ln: rows must be 16-byte aligned");
+    PIVP_REQUIRE(hd::a16(gamma) && hd::a16(beta) && (!y || (hd::a16(y) && y_cs % 4 == 0 && y_co % 4 == 0)), "heads_fwd_ln: rows must be 16-byte aligned");
     hd::LnIn ln{gamma, beta, reinterpret_cast<const float2*>(partial), (int)((long)HW * hd::C / 4096), eps, reinterpret_cast<float2*>(stats), y, y_cs, y_co};
     return heads_fwd_impl(x, x_cs, x_co, W, bias, out_a, Na, out_b, NH, B, HW, ln, stream);
 }

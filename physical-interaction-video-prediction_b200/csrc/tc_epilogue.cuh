@@ -21,7 +21,8 @@ struct TcEpilogue {
     int relu;                                    // mode 0: ReLU after bias
     int accumulate;                              // mode 0: out += D (fp32 view only)
     int atomic;                                  // mode 0: out += D with vector atomics (split-K CTAs of the halo kernel share an output tile)
-    float* gates;                                // mode 1: activated gates [M][N] (saved for backward); bf16 storage when gates_bf16
+    float* gates;                                // mode 1: activated gates [M][N] (saved for backward); bf16 storage when gates_bf16;
+                                                 //   null: not stored (the launchers then pick the instantiation without the gate store)
     int gates_bf16;
     float2* ln_partial;                          // per-tile (mean, M2) of the output for the LayerNorm that follows, 4096 values each:
     int ln_S;                                    //   mode 1 (halo kernel): partial[b * ln_S + tile_in_sample * (C / 32) + n_tile];
@@ -233,6 +234,9 @@ __device__ __forceinline__ void tc_epilogue_row_stage(const TcEpilogue& ep, uint
     }
 }
 
+// GATES = false (mode 1, pivp_tc_conv5x5 flags bit 2): the activated gates are not stored (forward-only prediction has no reader for them).
+// Each thread reads c_prev for exactly the (pixel, channel) elements it later writes to c_out, so c_prev may alias c_out.
+template <bool GATES = true>
 __device__ __forceinline__ void tc_epilogue_row(const TcEpilogue& ep, uint32_t trow, long m, long orow, int n0, int BN, int n_tile,
                                                 const float* bias_s) {
     if (ep.mode == 0) {
@@ -300,7 +304,8 @@ __device__ __forceinline__ void tc_epilogue_row(const TcEpilogue& ep, uint32_t t
                 hn[i] = (ep.accurate ? tanhf(cn[i]) : tanh_fast(cn[i])) * o;
                 gj[i] = j; gi[i] = ii; gf[i] = f; go[i] = o;
             }
-            if (ep.gates_bf16) {
+            if (!GATES) {
+            } else if (ep.gates_bf16) {
                 __nv_bfloat16* gb = reinterpret_cast<__nv_bfloat16*>(ep.gates) + m * (4 * ep.C) + n0 + c0;
                 *reinterpret_cast<uint4*>(gb) = pack8_bf16(gj);
                 *reinterpret_cast<uint4*>(gb + 32) = pack8_bf16(gi);

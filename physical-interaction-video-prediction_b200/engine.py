@@ -44,7 +44,9 @@ def _ptr(t):
 
 class Engine(object):
     def __init__(self, model_type="CDNA", num_masks=10, use_state=True, height=64, width=64, context_frames=2,
-                 device="cuda", compute="f32", stp_oob="zeros"):
+                 device="cuda", compute="f32", stp_oob="zeros", params=None):
+        """``params``: the flat parameter buffer of another engine of the same configuration, shared by reference (a forward-only engine:
+        the parameters are not re-initialised and no gradient buffer is allocated).  None: own parameters, LeCun-normal initialised."""
         if model_type not in ("CDNA", "DNA", "STP"):
             raise ValueError("No network specified")
         if model_type == "DNA" and num_masks != 1:
@@ -68,13 +70,20 @@ class Engine(object):
         self.cs3 = (64 + self.sa + 3) // 4 * 4          # row stride of the enc3 input [enc2 out | smear]: 74 channels in 76-float rows (16-B aligned)
         self.specs, self.nparam = layout.param_specs(model_type, self.M, self.use_state, self.H, self.W)
         self.spec = {s.name: s for s in self.specs}
+        self.ws = None
+        self.tc = None                                   # tensor-core (bf16) plan, created lazily
+        self.grad_sync = None                            # parallel.GradSync when the all-reduce is overlapped with the deferred weight gradients
+        if params is not None:
+            if params.numel() != self.nparam or params.dtype != torch.float32 or not params.is_cuda:
+                raise ValueError("params: a CUDA float32 buffer of %d parameters is required" % self.nparam)
+            self.flat_p, self.flat_g = params, None
+            self.p = {s.name: self.flat_p[s.offset:s.offset + s.size] for s in self.specs}
+            self.g = {}
+            return
         self.flat_p = torch.zeros(self.nparam, dtype=torch.float32, device=self.dev)
         self.flat_g = torch.zeros(self.nparam, dtype=torch.float32, device=self.dev)
         self.p = {s.name: self.flat_p[s.offset:s.offset + s.size] for s in self.specs}
         self.g = {s.name: self.flat_g[s.offset:s.offset + s.size] for s in self.specs}
-        self.ws = None
-        self.tc = None                                   # tensor-core (bf16) plan, created lazily
-        self.grad_sync = None                            # parallel.GradSync when the all-reduce is overlapped with the deferred weight gradients
         self.load_chainer_params(layout.lecun_normal_init(self.specs))
 
     # ------------------------------------------------------------------ parameters
@@ -412,9 +421,11 @@ class Engine(object):
             self.stage_schedule(take_gt)
         return self.forward_device(images, actions, states, feedself)
 
-    def forward_device(self, images, actions, states, feedself=True):
-        """Device part of the forward pass: stream-ordered work only (CUDA-graph capturable)."""
-        T, B = int(images.shape[0]), int(images.shape[1])
+    def forward_device(self, images, actions, states, feedself=True, steps=None, loss=True):
+        """Device part of the forward pass: stream-ordered work only (CUDA-graph capturable).
+        ``steps``: sequence length T when ``images`` holds the context frames only (feedself reads images[t] for t < context_frames);
+        ``loss=False``: no loss terms (states[0] is then the only state read)."""
+        T, B = int(images.shape[0]) if steps is None else int(steps), int(images.shape[1])
         H, W = self.H, self.W
         assert images.shape[2:] == (3, H, W) and images.dtype == torch.float32 and images.is_contiguous()
         ws = self._workspace(B, T)
@@ -423,7 +434,8 @@ class Engine(object):
         self.feedself = bool(feedself)
         self.images, self.states = images, states
         ws["cur"][0].copy_(states[0])
-        ws["loss_slots"].zero_()
+        if loss:
+            ws["loss_slots"].zero_()
         self.prev = []
         p = self.p
         n_img, n_sta = B * 3 * H * W, B * 5
@@ -552,6 +564,8 @@ class Engine(object):
                 L.call("pivp_stp_fused_fwd", _ptr(prev), _ptr(ws["enc7_pre"][t]), _ptr(ws["mask_pre"][t]), _ptr(ws["theta_raw"][t]),
                        _ptr(ws["gen"][t]), B, H, W, self.M, self.oob, s)
             # ---- loss terms of this step (train_model.py:737-758) on side branch 1: sums to loss_slots, loss gradients to d_gen / d_gs
+            if not loss:
+                continue
             with self._fork(1):
                 s1 = self._s()
                 if t >= self.ctx - 1:
@@ -562,7 +576,8 @@ class Engine(object):
                 else:
                     ws["d_gen"][t].zero_()
                     ws["d_gs"][t].zero_()
-        self._join(1)
+        if loss:
+            self._join(1)
         self.T, self.B = T, B
         return ws["gen"]
 

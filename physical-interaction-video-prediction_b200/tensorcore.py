@@ -17,6 +17,8 @@ from ._lib import PivpError
 
 
 class TensorCorePlan(object):
+    store_gates = True                                   # ConvLSTM forward keeps its activated gates (bf16, dg_bf16) for the backward pass
+
     def __init__(self, eng, ws):
         self.eng = eng
         self.ws = ws
@@ -334,8 +336,9 @@ class TensorCorePlan(object):
                  _ptr(self.dg_bf16[li][t]), _ptr(ws["c"][li][t - 1]) if t > 0 else 0, _ptr(ws["c"][li][t]),
                  _ptr(ws["xh"][li][t + 1]), cin + C, cin, _ptr(self.xh_bf16[li][t + 1]), self.Kpad[li], cin,
                  0, 0, 0,
-                 C, 1.0, self.accurate | 2, _ptr(ws["ln_ws"]) if self.ln_fused[li] else 0, e._s())
-        # flags bit 1: the activated gates are stored bf16, in dg_bf16[li][t]; ln_ws: LayerNorm statistics of h from the epilogue
+                 C, 1.0, self.accurate | (2 if self.store_gates else 4), _ptr(ws["ln_ws"]) if self.ln_fused[li] else 0, e._s())
+        # flags bit 1: the activated gates are stored bf16, in dg_bf16[li][t] (bit 2 instead: not stored); ln_ws: LayerNorm statistics of h
+        # from the epilogue
 
     def lstm_dgrad(self, li, t):
         """dxh = conv(dG_t, tap-flipped W): gradient w.r.t. the concatenated input [x | h_{t-1}] (D.5)."""
