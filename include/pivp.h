@@ -320,6 +320,35 @@ size_t pivp_tc_wgrad_workspace_bytes(int SB, int H, int W, int Cx, int N4);
 int pivp_tc_wgrad5x5(const void* dg_bf16, const void* xh_bf16, int xh_cs, int SB, int H, int W, int Cx, int N4, float* dW,
                      void* workspace, size_t ws_bytes, void* stream);
 
+/* ---- cross-entropy-method planning over the forward-only predictor (planner.py) -------------------------------------------------
+ * One iteration = sample -> predictor forward -> goal cost -> refit, all stream-ordered (graph-capturable), no host synchronisation.
+ * Shapes: actions (T-1, Bp, 5) with row stride Bp (the predictor's action buffer; step t of candidate n at (t*Bp + n)*5); the S = T - ctx
+ * sampled steps are t = ctx-1 .. T-2 (step s of the distribution is action step ctx-1+s); mean / std (S, 5); predicted frames
+ * gen (T-1, Bp, 3, H, W).  Bad arguments return PIVP_EINVAL before any CUDA call. */
+/* largest N pivp_cem_refit ranks (its bitonic sort keeps the N keys in shared memory) */
+int pivp_cem_max_samples(void);
+/* a[t, n, d] = clip(mean[s, d] + std[s, d] * eps, low[d], high[d]) for t = ctx-1+s, every one of the Bp rows n (padding rows included);
+ * rows t < ctx-1 are not written.  eps ~ N(0, 1): one Box-Muller pair from the Philox4x32-10 block of curand keyed by *seed (a device
+ * int64, read at run time: a new seed needs no new capture) at counter (e = (n*S + s)*5 + d, iteration), so a value depends on neither
+ * the launch geometry nor Bp.  std == 0 gives exactly clip(mean).  low / high: HOST arrays of 5 floats (read at the call, so baked into
+ * a captured graph), either may be NULL (no bound on that side); low[d] > high[d] or a NaN bound is PIVP_EINVAL. */
+int pivp_cem_sample(float* actions, int T, int Bp, int ctx, const float* mean, const float* std_, const float* low, const float* high,
+                    const long* seed, int iteration, void* stream);
+/* cost[n] = sum_t w[t] * mean_{c,y,x} (gen[t, n, c, y, x] - goal[t or 0, c, y, x])^2 for n < N (cost[n >= N] untouched).
+ * goal: one image (goal_per_step = 0) or T-1 images.  weights: device (T-1,); a step with w[t] == 0 is not read.  One CTA per row with a
+ * fixed reduction tree: the order depends only on (H, W, T), so the same frames give a bit-identical cost at any N and Bp.
+ * gen and goal must be 16-byte aligned (float4 loads) and 3*H*W a multiple of 4 (PIVP_EINVAL otherwise). */
+int pivp_goal_cost(const float* gen, int T, int Bp, int N, int H, int W, const float* goal, int goal_per_step, const float* weights,
+                   float* cost, void* stream);
+/* One CTA.  Ranks cost[0 .. N) by the 64-bit key (order-preserving float bits, index): ties go to the lower index, NaN after +inf.  The K
+ * lowest are the elites; per (s, d) their mean and population standard deviation (ddof 0, two passes, fixed order) give
+ *   mean <- alpha * mean + (1 - alpha) * elite_mean,  std <- max(alpha * std + (1 - alpha) * elite_std, min_std).
+ * Best-so-far record: when the lowest cost is strictly below *best_cost, *best_cost takes it and best_actions (T-1, 5) the candidate's
+ * whole action row (context steps included).  history[2*iteration .. +1] = (lowest cost, mean elite cost).
+ * Needs 1 <= K <= N <= min(Bp, pivp_cem_max_samples()), 0 <= alpha < 1, min_std >= 0, ctx >= 1, T - ctx >= 1. */
+int pivp_cem_refit(const float* cost, const float* actions, int T, int Bp, int ctx, int N, int K, float alpha, float min_std,
+                   float* mean, float* std_, float* best_cost, float* best_actions, float* history, int iteration, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -142,10 +142,11 @@ class ForwardEngine(Engine):
             self.tc = ForwardPlan(self, ws)
         return ws
 
-    def predict_device(self, context, actions, state0, T):
-        """context (>= min(T-1, context_frames), B, 3, H, W), actions (T-1, B, 5), state0 (1, B, 5): stream-ordered work only (capturable)."""
+    def predict_device(self, context, actions, state0, T, refresh=True):
+        """context (>= min(T-1, context_frames), B, 3, H, W), actions (T-1, B, 5), state0 (1, B, 5): stream-ordered work only (capturable).
+        ``refresh=False`` skips the bf16 weight refresh (a caller that runs several passes on unchanged parameters refreshes once)."""
         ws = self._workspace(int(context.shape[1]), int(T))
-        if self.tc is not None:
+        if self.tc is not None and refresh:
             self.tc.refresh_weights()                  # bf16 weight operands from the current flat_p: first node of a captured graph
         for li, (cin, c) in enumerate(zip(LSTM_IN, LSTM_SIZES)):
             ws["xh"][li][0][:, cin:].zero_()           # h_{-1} = 0: slot 0 of the ring held h of an odd step of the previous pass
